@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — env-steps/s of the batched Simulator.step() hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--envs E] [--map M]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--envs E] [--map M] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A "step" is one pass of the hot path over one batch: `env.step(actions)` for all E envs of the
@@ -159,10 +159,35 @@ def workload_text(c):
             f"distortion={c['distortion']}, device-side auto-reset")
 
 
-def run_config(c, K, Wm, rank, world, local_rank, obs_format="hwc_uint8", sampler=None, gather=True, gather_impl="fused"):
+DUMP_BYTES = 60_000_000   # below 64 MB in all, .npy headers included
+
+
+def dump_outputs(out_dir, obs, reward, done, info):
+    """Write what env.step() handed its caller -- obs, reward, done and every per-env array of info -- to
+    out_dir/<name>.npy: uint8 / bool / float32 as float32, wider types as float64, values unchanged.  When all envs do
+    not fit DUMP_BYTES, a fixed seeded sample of them is written and env_index.npy names the envs kept, so two builds
+    run with the same arguments can be compared array for array."""
+    import torch
+    arrays = {"obs": obs, "reward": reward, "done": done, **{f"info_{k}": v for k, v in info.items()}}
+    narrow = (torch.uint8, torch.bool, torch.float32)
+    per_env = 8 + sum(t[0].numel() * (4 if t.dtype in narrow else 8) for t in arrays.values())
+    E = obs.shape[0]
+    n = min(E, DUMP_BYTES // per_env)
+    idx = np.arange(E) if n == E else np.sort(np.random.default_rng(0).choice(E, n, replace=False))
+    sel = torch.from_numpy(idx).to(obs.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "env_index.npy"), idx.astype(np.float64))
+    for name, t in arrays.items():
+        t = t.index_select(0, sel).to(torch.float32 if t.dtype in narrow else torch.float64)
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.cpu().numpy())
+
+
+def run_config(c, K, Wm, rank, world, local_rank, obs_format="hwc_uint8", sampler=None, gather=True, gather_impl="fused",
+               dump_dir=None):
     """Device-resident arm of one workload: W warm-up steps, K timed steps (k_step_logic + render) bracketed by
-    barrier + synchronize, + the end-of-rollout NCCL all-gather when world > 1.  Returns (result dict, env) —
-    the env is left alive for the caller's end-to-end arm."""
+    barrier + synchronize, + the end-of-rollout NCCL all-gather when world > 1.  With dump_dir, the outputs of the
+    last timed step are written there (dump_outputs).  Returns (result dict, env) — the env is left alive for the
+    caller's end-to-end arm."""
     import torch
     import torch.distributed as dist
     from gym_duckietown_b200.batched_env import BatchedDuckietownEnv
@@ -224,11 +249,13 @@ def run_config(c, K, Wm, rank, world, local_rank, obs_format="hwc_uint8", sample
     for t in range(K):
         if fg is not None and t == K - 1:
             fg.arm()                              # the rollout's last step also fills every rank's gather buffer
-        env.step(actions[Wm + t])                 # dts_step: k_step_logic (+ device auto-reset) + the render kernels
+        out = env.step(actions[Wm + t])           # dts_step: k_step_logic (+ device auto-reset) + the render kernels
     if ag is not None:
         ag.all_gather(gathered)                   # baseline: the single end-of-rollout NCCL all-gather (SURVEY 8e)
     ev1.record()
     barrier()
+    if dump_dir is not None:
+        dump_outputs(dump_dir, *out)              # before the untimed steps below overwrite obs and state
     env.sim.profile(0)
     launches = env.launch_count() - launches0
     env.check()   # no frame hit a capacity limit
@@ -300,6 +327,8 @@ def main():
     ap.add_argument("--c4-envs", type=int, default=8192)
     ap.add_argument("--gather", default="fused", choices=["fused", "nccl"],
                     help="N>1: end-of-rollout observation exchange fused into the last step's rasteriser (peer memory), or NCCL")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write obs / reward / done / info of the headline's last timed step (rank 0) to DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -348,7 +377,8 @@ def main():
 
     # ---- device-resident arm: `value` -------------------------------------------------------------
     sampler = ClockSampler(local_rank) if rank == 0 else None
-    res, env = run_config(head, K, Wm, rank, world, local_rank, args.obs_format, sampler, gather_impl=args.gather)
+    res, env = run_config(head, K, Wm, rank, world, local_rank, args.obs_format, sampler, gather_impl=args.gather,
+                          dump_dir=args.dump_outputs if rank == 0 else None)
     config["gather"] = res.get("gather")
     if args.obs_format != "hwc_uint8":
         config["obs_format"] = args.obs_format

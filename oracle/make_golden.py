@@ -15,6 +15,10 @@ Files written
                        look-at, model-view of every draw, GL_LIGHT0 (eye-space position, ambient, diffuse), current
                        colour, bound texture, draw order; the vertex lists            (simulator.py:386-527, 564-586,
                        1707-1951; objects.py:123-148)
+  wrapper_interface.npz  observation spaces / shapes of the reference's PyTorchObsWrapper + ResizeWrapper around an
+                       object with the product Simulator's spaces                      (wrappers.py:93-141)
+  objmesh.npz          ObjMesh's extents and per-corner attributes for the synthetic OBJ of tests/test_obj_loader.py
+                       (objmesh.py:65-293)
 """
 from __future__ import annotations
 
@@ -466,6 +470,68 @@ def gen_wrappers(seed=21):
     print("wrappers:", sorted(out))
 
 
+def gen_wrapper_interface():
+    """The reference's PyTorchObsWrapper and ResizeWrapper (wrappers.py:93-141), unmodified, wrapped around an object
+    that carries the product Simulator's spaces and step / reset signature -> tests/golden/wrapper_interface.npz: the
+    observation spaces they declare and the shapes they return."""
+    refstub.install()
+    import importlib
+    W = importlib.import_module("gym_duckietown.wrappers")
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from test_reference_wrappers import StandIn
+
+    pt = W.PyTorchObsWrapper(StandIn())
+    first = pt.reset()
+    second = pt.step([0, 0])[0]
+    rz = W.ResizeWrapper(pt, resize_w=84, resize_h=84)
+    out = {"obs_shapes": np.array([first.shape, second.shape])}
+    for tag, sp in (("pytorch", pt.observation_space), ("resize", rz.observation_space)):
+        out[f"{tag}_shape"] = np.array(sp.shape)
+        out[f"{tag}_low"], out[f"{tag}_high"] = np.array(sp.low).ravel()[:1], np.array(sp.high).ravel()[:1]
+        out[f"{tag}_dtype"] = np.dtype(sp.dtype).str
+    out["resize_reset_shape"] = np.array(rz.reset().shape)
+    np.savez_compressed(os.path.join(OUT, "wrapper_interface.npz"), **out)
+    print("wrapper_interface:", {k: np.asarray(v).tolist() for k, v in out.items()})
+
+
+def gen_objmesh():
+    """The reference's ObjMesh loader (objmesh.py:65-293) on the synthetic OBJ / MTL pair of tests/test_obj_loader.py
+    -> tests/golden/objmesh.npz: extents and the per-corner attributes it hands pyglet."""
+    import tempfile
+    refstub.install()
+    import gym_duckietown.objmesh as M
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from test_obj_loader import MTL, OBJ, source_digest
+
+    captured = []
+
+    def vertex_list(n, *attrs):
+        captured.append({name: np.array(data, dtype=np.float32) for name, data in attrs})
+        return object()
+
+    with tempfile.TemporaryDirectory() as d:
+        for name, text in (("prop.obj", OBJ), ("prop.mtl", MTL)):
+            with open(os.path.join(d, name), "w") as f:
+                f.write(text)
+
+        def resource(name):
+            p = os.path.join(d, name)
+            if not os.path.exists(p):
+                raise KeyError(name)
+            return p
+
+        M.pyglet.graphics.vertex_list = vertex_list
+        M.get_resource_path = resource
+        ref = M.ObjMesh(os.path.join(d, "prop.obj"), "prop")
+    np.savez_compressed(
+        os.path.join(OUT, "objmesh.npz"), source_sha=source_digest(), min_coords=ref.min_coords, max_coords=ref.max_coords,
+        tri_pos=np.concatenate([c["v3f"].reshape(-1, 3, 3) for c in captured]),
+        tri_nrm=np.concatenate([c["n3f"].reshape(-1, 3, 3) for c in captured]),
+        tri_uv=np.concatenate([c["t2f"].reshape(-1, 3, 2) for c in captured]),
+        tri_col=np.concatenate([c["c3f"].reshape(-1, 3, 3) for c in captured]))
+    print(f"objmesh: {sum(len(c['v3f']) // 9 for c in captured)} triangles in {len(captured)} vertex lists")
+
+
 def gen_gltrace(name: str, seeds=(11, 12, 13), poses_per_episode=8, width=160, height=120):
     """Run the reference's render path against the recording GL (oracle/gltrace.py): reset() + a short walk, twice per
     seed (the second episode captures GL_LIGHT0 under the previous frame's model-view, S:581), domain_rand off and on."""
@@ -573,6 +639,11 @@ if __name__ == "__main__":
         os.makedirs(OUT, exist_ok=True)
         gen_wrappers()
         sys.exit(0)
+    if len(sys.argv) > 1 and sys.argv[1] == "interfaces":
+        os.makedirs(OUT, exist_ok=True)
+        gen_wrapper_interface()
+        gen_objmesh()
+        sys.exit(0)
     if len(sys.argv) > 1 and sys.argv[1] == "gltrace":
         os.makedirs(OUT, exist_ok=True)
         for m in MAPS:
@@ -592,5 +663,7 @@ if __name__ == "__main__":
     gen_reset_custom()
     gen_helpers()
     gen_wrappers()
+    gen_wrapper_interface()
+    gen_objmesh()
     for m in MAPS:
         gen_gltrace(m)

@@ -1,9 +1,8 @@
 """Stub-import harness: run the reference's OWN numpy arithmetic without its missing dependencies.
 
 TEST INFRASTRUCTURE ONLY.  Nothing in the product package imports this file.  It is used by
-``oracle/make_golden.py`` (in the build container, where ``/root/reference`` exists) to produce
-the fixtures under ``tests/golden/`` and by the ``not gpu`` tests that are skipped when the
-reference tree is absent (e.g. on the GPU box).
+``oracle/make_golden.py``, where the reference source tree is present, to produce the fixtures
+under ``tests/golden/``; the tests only read those fixtures.
 
 What it does (SURVEY.md appendix C): registers placeholder modules for pyglet / gym / geometry /
 duckietown_world / zuper_commons / carnivalmirror in ``sys.modules`` so that

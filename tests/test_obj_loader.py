@@ -1,16 +1,12 @@
 """assets.load_obj (Wavefront reader for real duckietown-world meshes) against the REFERENCE's ObjMesh loader
-(objmesh.py:65-293), executed through the stub-import harness on a synthetic OBJ/MTL pair.  Skipped where the
-reference tree is absent (GPU box)."""
+(objmesh.py:65-293) on a synthetic OBJ/MTL pair.  tests/golden/objmesh.npz holds what ObjMesh produced for this pair
+(`python oracle/make_golden.py interfaces`, which runs the reference through the stub-import harness)."""
+import hashlib
 import os
-import sys
 
 import numpy as np
-import pytest
 
-sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle"))
-import refstub  # noqa: E402
-
-pytestmark = pytest.mark.skipif(not refstub.reference_available(), reason="needs /root/reference")
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "objmesh.npz")
 
 OBJ = """# synthetic prop
 mtllib prop.mtl
@@ -40,33 +36,18 @@ Kd 0.1 0.2 0.9
 """
 
 
+def source_digest():
+    return hashlib.sha256((OBJ + MTL).encode()).hexdigest()
+
+
 def test_load_obj_matches_reference_objmesh(tmp_path):
     from gym_duckietown_b200 import assets
     (tmp_path / "prop.obj").write_text(OBJ)
     (tmp_path / "prop.mtl").write_text(MTL)
-    refstub.install()
-    import gym_duckietown.objmesh as M
-
-    captured = []
-
-    def vertex_list(n, *attrs):
-        captured.append({name: np.array(data, dtype=np.float32) for name, data in attrs})
-        return object()
-
-    def resource(name):
-        p = tmp_path / name
-        if not p.exists():
-            raise KeyError(name)
-        return str(p)
-
-    M.pyglet.graphics.vertex_list = vertex_list
-    M.get_resource_path = resource
-    ref = M.ObjMesh(str(tmp_path / "prop.obj"), "prop")
+    ref = np.load(GOLD)
+    assert str(ref["source_sha"]) == source_digest()      # the golden file was made from this very OBJ / MTL pair
     mine = assets.load_obj(str(tmp_path / "prop.obj"), "prop")
-    assert np.array_equal(mine.min_coords, ref.min_coords) and np.array_equal(mine.max_coords, ref.max_coords)
-    pos = np.concatenate([c["v3f"].reshape(-1, 3, 3) for c in captured])
-    nrm = np.concatenate([c["n3f"].reshape(-1, 3, 3) for c in captured])
-    uv = np.concatenate([c["t2f"].reshape(-1, 3, 2) for c in captured])
-    col = np.concatenate([c["c3f"].reshape(-1, 3, 3) for c in captured])
-    assert np.array_equal(mine.tri_pos, pos)      # incl. the max().min() re-centring quirk (objmesh.py:219)
-    assert np.array_equal(mine.tri_nrm, nrm) and np.array_equal(mine.tri_uv, uv) and np.array_equal(mine.tri_col, col)
+    assert np.array_equal(mine.min_coords, ref["min_coords"]) and np.array_equal(mine.max_coords, ref["max_coords"])
+    assert np.array_equal(mine.tri_pos, ref["tri_pos"])      # incl. the max().min() re-centring quirk (objmesh.py:219)
+    assert np.array_equal(mine.tri_nrm, ref["tri_nrm"]) and np.array_equal(mine.tri_uv, ref["tri_uv"])
+    assert np.array_equal(mine.tri_col, ref["tri_col"])

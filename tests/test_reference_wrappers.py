@@ -6,13 +6,16 @@ the numpy semantics the GPU tests rely on are those outputs.  GPU part (-m gpu):
 (dts_set_resize) against cv2.INTER_CUBIC as the reference wrapper called it."""
 import hashlib
 import os
-import sys
 
 import numpy as np
 import pytest
 
+from gym_duckietown_b200.gymshim import spaces
+from gym_duckietown_b200.simulator import Simulator
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLD = os.path.join(ROOT, "tests", "golden", "wrappers.npz")
+GOLD_INTERFACE = os.path.join(ROOT, "tests", "golden", "wrapper_interface.npz")
 
 
 def canned_frames(seed, h, w):
@@ -51,41 +54,62 @@ def test_reward_and_action_wrapper_semantics_are_the_reference_classes():
     assert np.array_equal(g["discrete_actions"], [[0.6, 1.0], [0.6, -1.0], [0.7, 0.0]])                   # DiscreteWrapper W:18-30
 
 
+class StandIn:
+    """The attributes gym_duckietown_b200.Simulator.__init__ sets (simulator.py) and its step / reset signature, without
+    CUDA: what a wrapper of the reference sees of the product env."""
+    metadata, reward_range = Simulator.metadata, (-1000, 1000)
+    action_space = spaces.Box(low=-1, high=1, shape=(2,), dtype=np.float32)
+    observation_space = spaces.Box(low=0, high=255, shape=(120, 160, 3), dtype=np.uint8)
+
+    @property
+    def unwrapped(self):
+        return self
+
+    def reset(self):
+        return np.zeros((120, 160, 3), np.uint8)
+
+    def step(self, a):
+        return np.ones((120, 160, 3), np.uint8), 0.0, False, {}
+
+
 def test_unmodified_reference_wrappers_accept_the_product_env_interface():
-    """The reference's wrappers.py, imported unmodified, wraps an object with the product Simulator's spaces and
-    step/reset signature and reproduces the PyTorchObsWrapper block of run_tests.py:28-34.  (Needs /root/reference;
-    the product env itself needs a GPU, so a shape-faithful stand-in carries its declared spaces here.)"""
-    sys.path.insert(0, os.path.join(ROOT, "oracle"))
-    import refstub
-    if not refstub.reference_available():
-        pytest.skip("reference tree not present")
-    refstub.install()
-    import importlib
-    Wm = importlib.import_module("gym_duckietown.wrappers")
-    import gym_duckietown_b200.simulator as PS
-    from gym_duckietown_b200.gymshim import spaces as pspaces
+    """The reference's wrappers.py, imported unmodified, wrapped StandIn in PyTorchObsWrapper and ResizeWrapper(84, 84)
+    as the PyTorchObsWrapper block of run_tests.py:28-34 does; tests/golden/wrapper_interface.npz holds the spaces and
+    shapes they returned.  StandIn must still offer what those wrappers read (W:96-103, 112-120: the observation
+    space's shape, dtype, low[0, 0, 0], high[0, 0, 0], high[1, 1, 1]; reset() and a 4-tuple step()) with the values
+    recorded, and the product's fused wrappers must declare the same spaces."""
+    from gym_duckietown_b200 import wrappers as PW
+    from gym_duckietown_b200.batched_env import BatchedDuckietownEnv
+    g = np.load(GOLD_INTERFACE)
+    env = StandIn()
+    sp = env.observation_space
+    assert [sp.shape[2], sp.shape[1], sp.shape[0]] == g["pytorch_shape"].tolist()
+    assert np.dtype(sp.dtype).str == str(g["pytorch_dtype"]) == str(g["resize_dtype"])
+    assert sp.low[0, 0, 0] == g["pytorch_low"][0] == g["resize_low"][0]
+    assert sp.high[0, 0, 0] == g["pytorch_high"][0] and sp.high[1, 1, 1] == g["resize_high"][0]
+    first, (second, _, _, _) = env.reset(), env.step([0, 0])
+    assert [first.T.shape, second.T.shape] == [tuple(s) for s in g["obs_shapes"]]      # observation(): transpose(2, 1, 0)
+    assert g["resize_shape"].tolist() == g["resize_reset_shape"].tolist() == [3, 84, 84]
 
-    class StandIn:   # the attributes gym_duckietown_b200.Simulator.__init__ sets (simulator.py), no CUDA
-        metadata, reward_range = PS.Simulator.metadata, (-1000, 1000)
-        action_space = pspaces.Box(low=-1, high=1, shape=(2,), dtype=np.float32)
-        observation_space = pspaces.Box(low=0, high=255, shape=(120, 160, 3), dtype=np.uint8)
+    class Batched:   # the part of BatchedDuckietownEnv the fused wrappers configure
+        camera_width, camera_height, resize = 160, 120, None
+        obs_size = BatchedDuckietownEnv.obs_size
 
-        @property
-        def unwrapped(self):
-            return self
+        def __init__(self):
+            self.output_format = dict(obs_layout="hwc", obs_dtype="uint8")
 
-        def reset(self):
-            return np.zeros((120, 160, 3), np.uint8)
+        def set_output_format(self, obs_layout=None, obs_dtype=None, **kw):
+            self.output_format.update({k: v for k, v in (("obs_layout", obs_layout), ("obs_dtype", obs_dtype)) if v})
 
-        def step(self, a):
-            return np.ones((120, 160, 3), np.uint8), 0.0, False, {}
+        def set_resize(self, w, h):
+            self.resize = (w, h)
 
-    env = Wm.PyTorchObsWrapper(StandIn())
-    first = env.reset()
-    second, _, _, _ = env.step([0, 0])
-    assert first.shape == tuple(env.observation_space.shape) == second.shape == (3, 160, 120)
-    rz = Wm.ResizeWrapper(env, resize_w=84, resize_h=84)
-    assert rz.reset().shape == (3, 84, 84)
+    pt = PW.PyTorchObsWrapper(Batched())
+    rz = PW.ResizeWrapper(PW.PyTorchObsWrapper(Batched()), resize_w=84, resize_h=84)
+    for tag, space in (("pytorch", pt.observation_space), ("resize", rz.observation_space)):
+        assert list(space.shape) == g[f"{tag}_shape"].tolist(), tag
+        assert np.dtype(space.dtype).str == str(g[f"{tag}_dtype"]), tag
+        assert space.low.flat[0] == g[f"{tag}_low"][0] and space.high.flat[0] == g[f"{tag}_high"][0], tag
 
 
 @pytest.mark.gpu
