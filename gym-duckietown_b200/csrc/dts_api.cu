@@ -440,8 +440,10 @@ int dts_set_fisheye_lut(dts_sim* sim, const float* rmapx, const float* rmapy, in
   for (int y = 0; y < H; y++)
     for (int x = 0; x < W; x++) {
       const float fx = rmapx[(size_t)y * W + x], fy = rmapy[(size_t)y * W + x];
-      const int sx = (int)rintf(fx), sy = (int)rintf(fy);   // round-half-even like the kernel's rintf
-      const bool ok = fx == fx && fy == fy && sx >= 0 && sx < W && sy >= 0 && sy < H;
+      // NaN, +-inf and |v| >= 2^31 have no int value (the cast would be undefined): such entries point outside
+      const bool finite = fabsf(fx) < 2147483648.0f && fabsf(fy) < 2147483648.0f;
+      const int sx = finite ? (int)rintf(fx) : -1, sy = finite ? (int)rintf(fy) : -1;   // round-half-even like the kernel's rintf
+      const bool ok = sx >= 0 && sx < W && sy >= 0 && sy < H;
       src[(size_t)y * W + x] = ok ? (int32_t)((uint32_t)(sx & 0xffff) | ((uint32_t)sy << 16)) : (int32_t)0x80008000u;
       if (!ok) continue;
       const int cb = (y / 8) * cbx_n + x / 32, f = ((y & 7) >> 2) * 4 + ((x & 31) >> 3);

@@ -556,9 +556,14 @@ void orr_render(const orr_scene* sc, double px, double pz, double angle, const o
     for (int xx = 0; xx < W; xx++) {
       int sx = xx, sy = y, valid = 1;
       if (lut_x) {
-        sx = (int)rintf(lut_x[(size_t)y * W + xx]);
-        sy = (int)rintf(lut_y[(size_t)y * W + xx]);
-        valid = sx >= 0 && sx < W && sy >= 0 && sy < H;  /* cv2.remap BORDER_CONSTANT -> 0 */
+        const float fx = lut_x[(size_t)y * W + xx], fy = lut_y[(size_t)y * W + xx];
+        /* NaN, +-inf and |v| >= 2^31 have no int value (the cast would be undefined): outside */
+        valid = fabsf(fx) < 2147483648.0f && fabsf(fy) < 2147483648.0f;
+        if (valid) {
+          sx = (int)rintf(fx);
+          sy = (int)rintf(fy);
+          valid = sx >= 0 && sx < W && sy >= 0 && sy < H;  /* cv2.remap BORDER_CONSTANT -> 0 */
+        }
       }
       for (int ch = 0; ch < 3; ch++) {
         uint8_t v = 0;

@@ -107,7 +107,8 @@ def test_fisheye_fused_gather_vs_oracle(torch_cuda):
         undist = sc.render(st["pos_x"][k], st["pos_z"][k], st["angle"][k], oracle_episode(orc, captured, k), W, H, True)
         assert np.array_equal(env.camera_model.distort(undist), cpu)   # oracle gather == product's numpy gather
         d = np.abs(gpu[k].astype(int) - cpu.astype(int))
-        assert d.max() <= 1, (k, d.max(), int((d > 1).sum()))
+        assert d.max() == 0, (k, d.max(), int((d > 0).sum()))
+    env.check()
     env.close()
 
 
