@@ -26,7 +26,6 @@
 //
 // HBM traffic per env-frame: obs store W*H*3 B (compulsory) + PrimRec slab / BinRec lists / lattice table
 // (tens of KB per env, written by k_geometry / k_bin and read once by k_raster) + texels (shared, L2-resident).
-#include <cstdlib>
 #include <cstddef>
 
 #include "dts_camera.cuh"
@@ -36,21 +35,6 @@ namespace dts {
 
 namespace {
 
-#ifndef DTS_RENDER_THREADS
-#define DTS_RENDER_THREADS 256
-#endif
-#ifndef DTS_RENDER_MIN_CTAS
-#define DTS_RENDER_MIN_CTAS 3
-#endif
-#ifndef DTS_TMA_STAGING
-#define DTS_TMA_STAGING 1   // 0: stage BinRec chunks with per-lane 128-bit loads + shared stores instead of cp.async.bulk (A/B switch)
-#endif
-#ifndef DTS_TINY_PATH
-#define DTS_TINY_PATH 1     // triangles whose pixel box inside a coarse bin is <= 4x4 are rasterised one per lane (A/B switch)
-#endif
-#ifndef DTS_SAMPLE_CULL
-#define DTS_SAMPLE_CULL 1   // triangles of at most 3x3 pixels that cover no sample position are dropped at set-up (A/B switch)
-#endif
 #ifndef DTS_STATS
 #define DTS_STATS 0         // 1: k_raster counts bins / prim visits / shading rounds into the diagnostic counters (tools/raster_stats.py)
 #endif
@@ -59,21 +43,9 @@ namespace {
 #else
 #define DTS_COUNT(slot, n) do { } while (0)
 #endif
-#ifndef DTS_SOLO
-#define DTS_SOLO 1          // coarse bins lying inside ONE prim (besides the ground) are drawn by the lean k_raster_solo (A/B switch)
-#endif
-#ifndef DTS_SOLO_MIN_CTAS
-#define DTS_SOLO_MIN_CTAS 3   // resident CTAs per SM of k_raster_solo (register budget 65536 / (256 * this))
-#endif
-#ifndef DTS_COPLANAR
-#define DTS_COPLANAR 1      // fine bins whose prims are all road tiles (coplanar, disjoint) resolve visibility by coverage alone (A/B switch)
-#endif
-#ifndef DTS_COARSE_FAST
-#define DTS_COARSE_FAST 0   // 1: coarse bins lying inside one prim skip visibility and fetch the prim once.  Measured
-                            // (profiles/README.md, r2d): +5 % k_raster time — the extra code and registers cost more
-                            // than the skipped flag tests save; kept as an A/B switch only
-#endif
-constexpr int kThreads = DTS_RENDER_THREADS;
+constexpr int kThreads = 256;       // k_raster CTA
+constexpr int kRenderMinCtas = 3;   // resident CTAs per SM of k_raster (register budget 65536 / (kThreads * this))
+constexpr int kSoloMinCtas = 3;     // resident CTAs per SM of k_raster_solo (register budget 65536 / (256 * this))
 constexpr int kWarps = kThreads / 32;
 constexpr int kBinW = 8, kBinH = 4;   // fine bin = one warp's pixel block (one pixel per lane)
 constexpr int kCFX = 4, kCFY = 2;     // coarse bin = 4 x 2 fine bins = 32 x 8 px: unit of binning and staging
@@ -86,39 +58,30 @@ constexpr int kSub = 64;          // sub-pixel units per pixel
 __host__ __device__ constexpr int sample_x(int s) { return s == 0 ? 24 : (s == 1 ? 56 : (s == 2 ? 8 : 40)); }
 __host__ __device__ constexpr int sample_y(int s) { return s == 0 ? 8 : (s == 1 ? 24 : (s == 2 ? 40 : 56)); }
 
-struct Vtx { float cx, cy, cz, cw, r, g, b, u, v; };
+// Fine bins of coarse bin (cbx, cby) that lie inside a W x H image: all 4 x 2 except on the right / bottom border.
+// k_bin hands a bin to k_raster_solo only if its prim covers every one of them; k_raster then skips the bin and
+// k_raster_solo draws exactly these fine bins, so all three take them from here.  As bit masks, bit f = fine bin
+// (f & 3, f >> 2): fine_bins_inside = row mask & column mask (k_raster keeps the row mask for a whole row of bins).
+__device__ __forceinline__ int fine_cols_in_image(int cbx, int W) { return min(kCFX, (W - cbx * kCoarseW + kBinW - 1) / kBinW); }   // 1..4
+__device__ __forceinline__ unsigned fine_col_mask(int cbx, int W) {
+  const unsigned cols = (1u << fine_cols_in_image(cbx, W)) - 1u;
+  return cols | (cols << 4);
+}
+__device__ __forceinline__ unsigned fine_row_mask(int cby, int H) { return ((cby * kCFY + 1) * kBinH < H) ? 0xffu : 0x0fu; }
+__device__ __forceinline__ unsigned fine_bins_inside(int cbx, int cby, int W, int H) { return fine_row_mask(cby, H) & fine_col_mask(cbx, W); }
 
-#ifndef DTS_GEO_X
-#define DTS_GEO_X 0   // code-size experiments of the geometry pass: bit 0 process_triangle_uniform out of line, bit 1 lattice loop rolled, bit 2 mesh vertex loop rolled
-#endif
-#ifndef DTS_GEO_INLINE
-#define DTS_GEO_INLINE 5
-#endif
-// which of the geometry pass's big device functions are inlined: bit 0 shade_vertex, bit 1 setup_and_emit, bit 2 the clipper.
-// The kernel is instruction-fetch bound (ncu: 6.9 stall_no_instruction cycles per issue, 174 KB of SASS against a 32 KB
-// L1.5 I-cache): with everything inlined setup_and_emit alone is 107 KB in a dozen copies.  Measured k_geometry at c2 / c3:
-// 7 (all inline) 198 / 466 us, 5 (one copy of setup_and_emit) 177 / 424 us, 1: 188 / 435, 3: 220 / 493, 0: 221 / 447.
-#define DTS_GEO_FN_SHADE __forceinline__
-#define DTS_GEO_FN_SETUP __forceinline__
-#define DTS_GEO_FN_CLIP __forceinline__
-#if !(DTS_GEO_INLINE & 1)
-#undef DTS_GEO_FN_SHADE
-#define DTS_GEO_FN_SHADE __noinline__
-#endif
-#if !(DTS_GEO_INLINE & 2)
-#undef DTS_GEO_FN_SETUP
-#define DTS_GEO_FN_SETUP __noinline__
-#endif
-#if !(DTS_GEO_INLINE & 4)
-#undef DTS_GEO_FN_CLIP
-#define DTS_GEO_FN_CLIP __noinline__
-#endif
-#ifndef DTS_GEO_WARPS
-#define DTS_GEO_WARPS 1
-#endif
-#ifndef DTS_GEO_MIN_CTAS
-#define DTS_GEO_MIN_CTAS 32
-#endif
+// The fisheye LUT entry of output pixel (x, y) (FishTab::src_xy, built by dts_set_fisheye_lut): the source pixel, in
+// sub-pixels, and whether it lies inside the image (cv2.remap BORDER_CONSTANT: black if not).  x, y are clamped to the
+// image, so lanes past its edge read an edge entry; their pixels are not stored.
+struct FishSrc { int x, y; bool valid; };
+__device__ __forceinline__ FishSrc fish_src(const FishTab& ft, int x, int y, int W, int H) {
+  const int gx = min(x, W - 1), gy = min(y, H - 1);
+  const int sxy = __ldg(ft.src_xy + gy * W + gx);
+  const int sx = (int)(short)(sxy & 0xffff), sy = sxy >> 16;
+  return {sx * kSub, sy * kSub, sx != -32768};
+}
+
+struct Vtx { float cx, cy, cz, cw, r, g, b, u, v; };
 
 struct __align__(16) PrimRec {   // 128 B in the env's slab, words grouped for 128-bit loads
   int32_t X0, Y0, X1, Y1;        // w0  snapped vertices in cyclic order, orientation normalised (area > 0)
@@ -189,8 +152,8 @@ __device__ __forceinline__ void model_view(const double* V, double tx, double ty
 }
 
 // fixed-function transform & lighting of one vertex (float32, operation order = spec)
-__device__ DTS_GEO_FN_SHADE Vtx shade_vertex(const Xform& x, const Shared& sh, float px, float py, float pz, float nx,
-                                            float ny, float nz, float cr, float cg, float cb, float u, float v) {
+__device__ __forceinline__ Vtx shade_vertex(const Xform& x, const Shared& sh, float px, float py, float pz, float nx,
+                                           float ny, float nz, float cr, float cg, float cb, float u, float v) {
   float e[3], ne[3];
 #pragma unroll
   for (int r = 0; r < 3; r++) {
@@ -278,8 +241,12 @@ struct EmitCtx {
 // With `d` the prim is the QUAD a,b,c,d (spec tile mode 1: an unclipped road tile): planes of triangle (a,b,c),
 // coverage by four edges.  Returns false — nothing emitted — if the snapped quad is not strictly convex; the
 // caller then draws the two triangles (a,b,c)(a,c,d) instead.
-__device__ DTS_GEO_FN_SETUP bool setup_and_emit(const EmitCtx& ec, const Vtx& a, const Vtx& b, const Vtx& c, int id,
-                                               int tex, int lat, const Vtx* d = nullptr) {
+// Out of line, while shade_vertex and the clipper are inlined: k_geometry is instruction-fetch bound (ncu: 6.9
+// stall_no_instruction cycles per issue, 174 KB of SASS against a 32 KB L1.5 I-cache), and inlined, setup_and_emit alone
+// is 107 KB in a dozen copies.  Measured k_geometry at c2 / c3 for each choice of inlined functions: all three 198 / 466 us,
+// shade_vertex + clipper (this) 177 / 424 us, shade_vertex 188 / 435, shade_vertex + setup_and_emit 220 / 493, none 221 / 447.
+__device__ __noinline__ bool setup_and_emit(const EmitCtx& ec, const Vtx& a, const Vtx& b, const Vtx& c, int id,
+                                            int tex, int lat, const Vtx* d = nullptr) {
   const Vtx* vs[3] = {&a, &b, &c};
   int X[3], Y[3];
   float zw[3], q[3];
@@ -319,7 +286,6 @@ __device__ DTS_GEO_FN_SETUP bool setup_and_emit(const EmitCtx& ec, const Vtx& a,
   const int px0 = max(minx >> 6, 0), px1 = min(maxx >> 6, ec.W - 1);
   const int py0 = max(miny >> 6, 0), py1 = min(maxy >> 6, ec.H - 1);
   if (px0 > px1 || py0 > py1) return true;   // off screen: emitted nothing, and nothing is what it covers
-#if DTS_SAMPLE_CULL
   if (!d && (maxx >> 6) - (minx >> 6) < 3 && (maxy >> 6) - (miny >> 6) < 3) {   // (the unclamped box: everything below stays small)
     // A small triangle that covers NO sample position draws nothing — half the triangles of a distant mesh at
     // 160x120 — so it needs no record, no bin pair and no visit by the rasteriser.  Same integer edge functions and
@@ -344,7 +310,6 @@ __device__ DTS_GEO_FN_SETUP bool setup_and_emit(const EmitCtx& ec, const Vtx& a,
       }
     if (!any) return true;
   }
-#endif
   PrimRec r;
   r.X0 = x0; r.Y0 = y0; r.X1 = x1; r.Y1 = y1; r.X2 = x2; r.Y2 = y2; r.X3 = x0; r.Y3 = y0;
   const float dx1 = (float)(x1 - x0) * 0.015625f, dy1 = (float)(y1 - y0) * 0.015625f;
@@ -403,7 +368,7 @@ __device__ __forceinline__ Vtx clip_lerp(const Vtx& in, const Vtx& out, float di
 // WHOLE warp for one triangle: lane k owns polygon vertex k, neighbours' plane distances come by shuffle, output
 // slots by ballot prefix sums, so a plane costs a few dozen instructions instead of a serial loop over vertices.
 // Same arithmetic, same vertex order (hence the same fan) as the serial formulation of the spec.
-__device__ DTS_GEO_FN_CLIP void clip_and_emit_warp(const EmitCtx& ec, const Vtx& a, const Vtx& b, const Vtx& c, int id,
+__device__ __forceinline__ void clip_and_emit_warp(const EmitCtx& ec, const Vtx& a, const Vtx& b, const Vtx& c, int id,
                                                    int tex, int lat, int lane) {
   for (int p2 = 0; p2 < 6; p2++) {   // the spec's trivial reject looks at the ORIGINAL triangle, guard planes
     const int cnt = !(plane_dist(a, p2) >= 0.0f) + !(plane_dist(b, p2) >= 0.0f) + !(plane_dist(c, p2) >= 0.0f);
@@ -446,13 +411,8 @@ __device__ DTS_GEO_FN_CLIP void clip_and_emit_warp(const EmitCtx& ec, const Vtx&
 }
 
 // one warp-uniform triangle (ground, analytic tile): classify once, lane 0 emits or the warp clips
-#if DTS_GEO_X & 1
-#define DTS_PTU_FN __noinline__
-#else
-#define DTS_PTU_FN __forceinline__
-#endif
-__device__ DTS_PTU_FN void process_triangle_uniform(const EmitCtx& ec, const Vtx& a, const Vtx& b, const Vtx& c,
-                                                    int id, int tex, int lat, int lane) {
+__device__ __forceinline__ void process_triangle_uniform(const EmitCtx& ec, const Vtx& a, const Vtx& b, const Vtx& c,
+                                                         int id, int tex, int lat, int lane) {
   const int cls = classify(a, b, c);
   if (cls == 2) return;
   if (cls == 0) { if (lane == 0) setup_and_emit(ec, a, b, c, id, tex, lat); }
@@ -566,7 +526,7 @@ __device__ __forceinline__ unsigned build_binrec(const PrimRec* __restrict__ pr,
     }
   }
   int tiny = 0;
-  if (DTS_TINY_PATH && !fb && !quad && live) {
+  if (!fb && !quad && live) {
     // small triangles (a 6 cm duckie is 148 triangles in a dozen pixels) are rasterised one per LANE in k_raster instead
     // of one per warp: they carry their pixel box
     const int minx = min(qx[0], min(qx[1], qx[2])) - ox, maxx = max(qx[0], max(qx[1], qx[2])) - ox;
@@ -805,7 +765,7 @@ __device__ __forceinline__ void store_bin_any(uint8_t* __restrict__ out, int fmt
 }  // namespace
 
 
-int render_ctas_per_sm() { return DTS_RENDER_MIN_CTAS; }
+int render_ctas_per_sm() { return kRenderMinCtas; }
 
 // ------------------------------------------------------------------------------------------------ frame memory
 struct FrameMem {
@@ -958,7 +918,7 @@ __global__ void __launch_bounds__(256) k_cull(const DState S, const DMap* __rest
 // ------------------------------------------------------------------------------------------------ k_geometry
 // One warp per CTA, 64 registers, 32 CTAs per SM: the kernel is latency-bound (short dependent chains), so resident warps
 // matter more than spills.  Each warp draws the (env, item) pairs of k_cull's work list, grid-strided.
-constexpr int kGeoWarps = DTS_GEO_WARPS;
+constexpr int kGeoWarps = 1, kGeoMinCtas = 32;
 template <bool kTess>   // true: spec tile mode 0 (DTS_FLAG_TESSELLATE), the literal 98 triangles per road tile
 __device__ __forceinline__ void geometry_item(const DState& S, const DMap* __restrict__ maps, const RenderCfg& rc, const FrameMem& fm,
                                               int max_prims, int max_lat, int32_t* __restrict__ err, int env, int item, int lane,
@@ -1027,11 +987,7 @@ __device__ __forceinline__ void geometry_item(const DState& S, const DMap* __res
     // the tile's 8x8 lattice, two vertices per lane (tessellated mode: also frustum-culls the whole tile)
     Vtx lv[2];
     int outside[6] = {0, 0, 0, 0, 0, 0};
-#if DTS_GEO_X & 2
-#pragma unroll 1
-#else
 #pragma unroll
-#endif
     for (int h = 0; h < 2; h++) {
       const int vi = lane + 32 * h, a = vi >> 3, b = vi & 7;             // a: u index (x), b: v index (z)
       const float lx = (float)(-ts / 2 + ((double)a / 7.0) * ts), lz = (float)(-ts / 2 + ((double)b / 7.0) * ts);
@@ -1130,7 +1086,7 @@ __device__ __forceinline__ void geometry_item(const DState& S, const DMap* __res
 }
 
 template <bool kTess>
-__global__ void __launch_bounds__(kGeoWarps * 32, DTS_GEO_MIN_CTAS)
+__global__ void __launch_bounds__(kGeoWarps * 32, kGeoMinCtas)
 k_geometry(const DState S, const DMap* __restrict__ maps, RenderCfg rc, FrameMem fm, int max_prims, int max_lat,
            int32_t* __restrict__ err) {
   __shared__ GeoWarp gws[kGeoWarps];
@@ -1293,7 +1249,7 @@ k_bin(RenderCfg rc, FrameMem fm, FishTab ft, int max_prims, int max_pairs, int32
   // pass 2: one pair per thread -> its visibility record (the pairs were written by other threads of this CTA: the
   // barrier above orders those writes before these reads)
   const int pair0 = s_base, total = s_total;
-  const bool solo_on = DTS_SOLO && rc.obs_layout == DTS_OBS_HWC && rc.obs_dtype == DTS_OBS_U8 && (W & 3) == 0;
+  const bool solo_on = rc.obs_layout == DTS_OBS_HWC && rc.obs_dtype == DTS_OBS_U8 && (W & 3) == 0;
   BinRec* recs = fm.recs;
   for (int i = pair0 + tid; i < pair0 + total; i += nthr) {
     const uint32_t pair = pairs[i];
@@ -1311,8 +1267,7 @@ k_bin(RenderCfg rc, FrameMem fm, FishTab ft, int max_prims, int max_pairs, int32
         // the coarse bin lies inside this prim and holds no other (besides the ground, hidden below it): no visibility
         // work at all -> the bin goes to k_raster_solo, and k_raster skips it (negative count)
         const int c = cnt[b];
-        const int nx = min(kCFX, (W - cbx * kCoarseW + kBinW - 1) / kBinW);
-        const unsigned cols = (1u << nx) - 1u, valid = (((cby * kCFY + 1) * kBinH < H) ? 0xffu : 0x0fu) & (cols | (cols << 4));
+        const unsigned valid = fine_bins_inside(cbx, cby, W, H);
         // (... or it is the bin's only record: a stretch of bare ground)
         const bool alone = (r & 0x100u) ? (c & kCountMask) == 1 : (c & kCountMask) - (c >> 20) == 1;
         if (alone && (r & valid) == valid) {
@@ -1362,7 +1317,7 @@ __device__ __forceinline__ float key_float(unsigned k) { return __uint_as_float(
 // ------------------------------------------------------------------------------------------------ k_raster
 template <bool kWrapFmt, bool kFish>   // kWrapFmt: a dts_output_format other than packed u8 HWC is written by the resolve;
                                        // kFish: every lane renders the SOURCE pixel the fisheye LUT names for its output pixel
-__global__ void __launch_bounds__(kThreads, DTS_RENDER_MIN_CTAS)
+__global__ void __launch_bounds__(kThreads, kRenderMinCtas)
 k_raster(const DState S, const DMap* __restrict__ maps, RenderCfg rc, FrameMem fm, FishTab ft, GatherTab gt,
          uint8_t* __restrict__ obs, int max_prims, int max_pairs, int max_lat, int32_t* __restrict__ err) {
   // dynamic shared memory (kRasterSmem bytes): per warp two chunks of records in flight, their mbarriers, and a 128-sample
@@ -1432,17 +1387,12 @@ k_raster(const DState S, const DMap* __restrict__ maps, RenderCfg rc, FrameMem f
       my_start = fm.bin_start[(size_t)env * cbins + cby * cbins_x + lane];
     }
     const unsigned nz = __ballot_sync(0xffffffffu, my_cnt > 0);
-    const unsigned fvalid_y = ((cby * kCFY + 1) * kBinH < H) ? 0xffu : 0x0fu;   // second row of fine bins inside the image?
+    const unsigned fvalid_y = fine_row_mask(cby, H);
     // ---- producer: walks the row's chunk sequence one chunk ahead of the consumer.  A list of <= 32 records is
     // ONE chunk shared by the bin's 8 fine bins; a longer list is streamed chunk by chunk for each fine bin in turn
     // (the records are ready-made, re-reading them from L2 costs no arithmetic).
     int pcbx = nz ? __ffs(nz) - 1 : 32, pf = 0, pc = 0;
-    // fine bins of coarse bin `cbx` that lie inside the image, as a bit mask (all 8 except on the right / bottom border)
-    auto valid8 = [&](int cbx) -> unsigned {
-      const int nx = min(kCFX, (W - cbx * kCoarseW + kBinW - 1) / kBinW);   // fine-bin columns inside the image: 1..4
-      const unsigned cols = (1u << nx) - 1u;
-      return fvalid_y & (cols | (cols << 4));
-    };
+    auto valid8 = [&](int cbx) -> unsigned { return fvalid_y & fine_col_mask(cbx, W); };   // fine_bins_inside(cbx, cby, W, H)
     auto fine_valid = [&](int cbx, int f) -> bool { return (valid8(cbx) >> f) & 1u; };
     auto next_bin = [&]() {
       const unsigned rem = nz & ~((2u << pcbx) - 1u);
@@ -1455,19 +1405,10 @@ k_raster(const DState S, const DMap* __restrict__ maps, RenderCfg rc, FrameMem f
       if (n > kStage) while (pf < kCFX * kCFY && !fine_valid(pcbx, pf)) pf++;   // fine bins outside the image are not visited
       if (n > kStage && pf >= kCFX * kCFY) { next_bin(); return; }               // (cannot happen: fine bin 0 is always inside)
       const int nch = min(kStage, n - pc);
-#if DTS_TMA_STAGING
       if (lane == 0) {
         mbar_expect_tx(&bar[ps], (uint32_t)(nch * sizeof(BinRec)));
         bulk_load(stages[warp][ps], recs + st + pc, (uint32_t)(nch * sizeof(BinRec)), &bar[ps]);
       }
-#else
-      if (lane < nch) {   // A/B baseline: one record per lane through registers
-        const int4* src = reinterpret_cast<const int4*>(recs + st + pc + lane);
-        int4* dst = reinterpret_cast<int4*>(&stages[warp][ps][lane]);
-#pragma unroll
-        for (int k = 0; k < 5; k++) dst[k] = __ldg(src + k);
-      }
-#endif
       ps ^= 1;
       if (n <= kStage) { next_bin(); return; }
       pc += kStage;
@@ -1489,10 +1430,8 @@ k_raster(const DState S, const DMap* __restrict__ maps, RenderCfg rc, FrameMem f
         for (int f = 0; f < kCFX * kCFY; f++)
           if ((fvalid >> f) & 1u) {
             unsigned rgb = clear_rgb;
-            if (kFish) {
-              const int gx = min((cbx * kCFX + (f & 3)) * kBinW + (lane & 7), W - 1), gy = min((cby * kCFY + (f >> 2)) * kBinH + (lane >> 3), H - 1);
-              if ((short)(__ldg(ft.src_xy + gy * W + gx) & 0xffff) == -32768) rgb = 0u;
-            }
+            if (kFish && !fish_src(ft, (cbx * kCFX + (f & 3)) * kBinW + (lane & 7), (cby * kCFY + (f >> 2)) * kBinH + (lane >> 3), W, H).valid)
+              rgb = 0u;
             emit(rgb, cbx * kCFX + (f & 3), cby * kCFY + (f >> 2));
           }
         continue;
@@ -1513,12 +1452,8 @@ k_raster(const DState S, const DMap* __restrict__ maps, RenderCfg rc, FrameMem f
           // ---- acquire this chunk; the next one starts loading into the other slot meanwhile
           __syncwarp();   // every lane is done with the slot the producer is about to refill
           issue();
-#if DTS_TMA_STAGING
           mbar_wait(&bar[cs], (parity >> cs) & 1u);
           parity ^= 1u << cs;
-#else
-          __syncwarp();
-#endif
           const BinRec* stage = stages[warp][cs];
           cs ^= 1;
           const int nch = min(kStage, count - c0);
@@ -1527,7 +1462,7 @@ k_raster(const DState S, const DMap* __restrict__ maps, RenderCfg rc, FrameMem f
           const bool first = c0 == 0, last = c0 + kStage >= count;
           const unsigned ground_bits = __ballot_sync(0xffffffffu, (mine.y & 2u) != 0u);   // the ground quad's records in this chunk
           const unsigned tiny_bits = kFish ? 0u : __ballot_sync(0xffffffffu, (mine.y & 4u) != 0u);   // one-per-lane triangles
-          const unsigned flat_bits = DTS_COPLANAR ? __ballot_sync(0xffffffffu, (mine.y & 8u) != 0u) : 0u;   // road tiles (plane y = 0)
+          const unsigned flat_bits = __ballot_sync(0xffffffffu, (mine.y & 8u) != 0u);   // road tiles (plane y = 0)
 #if DTS_STATS
           if (single) {   // census: coarse bins lying inside ONE prim (besides the ground)
             const unsigned ng_ = __ballot_sync(0xffffffffu, !(mine.y & 2u) && ((mine.x >> 16) & fvalid) != 0u);
@@ -1535,47 +1470,16 @@ k_raster(const DState S, const DMap* __restrict__ maps, RenderCfg rc, FrameMem f
             if (ng_ && !(ng_ & (ng_ - 1)) && (ng_ & ngfull_)) { DTS_COUNT(22, 1); DTS_COUNT(23, __popc(fvalid)); }
           }
 #endif
-          if (DTS_COARSE_FAST && single) {
-            // ---- the whole coarse bin lies inside ONE prim (besides the ground quad, hidden below it): no visibility
-            // work at all, the prim's planes are fetched once for the bin's 256 pixels
-            const unsigned ng = __ballot_sync(0xffffffffu, !(mine.y & 2u) && ((mine.x >> 16) & fvalid) != 0u);
-            const unsigned ngfull = __ballot_sync(0xffffffffu, !(mine.y & 2u) && ((mine.x >> 24) & fvalid) == fvalid);
-            if (ng && !(ng & (ng - 1)) && (ng & ngfull)) {
-              const ShadeIn si = load_shade(prims, stage[__ffs(ng) - 1].prim_flags & 0xffffu);
-#pragma unroll 1
-              for (int f = 0; f < kCFX * kCFY; f++) {
-                if (!((fvalid >> f) & 1u)) continue;
-                const int bx = cbx * kCFX + (f & 3), by = cby * kCFY + (f >> 2);
-                int pxa = ox + pxs + (f & 3) * kBinW * kSub, pya = oy + pys + (f >> 2) * kBinH * kSub;
-                bool px_valid = true;
-                if (kFish) {
-                  const int gx = min(bx * kBinW + (lane & 7), W - 1), gy = min(by * kBinH + (lane >> 3), H - 1);
-                  const int sxy = __ldg(ft.src_xy + gy * W + gx);
-                  const int sx = (int)(short)(sxy & 0xffff), sy = sxy >> 16;
-                  px_valid = sx != -32768;
-                  pxa = sx * kSub; pya = sy * kSub;
-                }
-                float c3[3];
-                shade_eval(si, tex_pool, lat_tab, pxa, pya, c3);
-                unsigned rgb = pack_rgb(c3[0], c3[1], c3[2]);
-                if (kFish && !px_valid) rgb = 0u;
-                emit(rgb, bx, by);
-              }
-              continue;
-            }
-          }
 #pragma unroll 1
           for (int f = (single ? 0 : g); f < (single ? kCFX * kCFY : g + 1); f++) {
             if (!((fvalid >> f) & 1u)) continue;
             const int bx = cbx * kCFX + (f & 3), by = cby * kCFY + (f >> 2);   // fine bin
             int pxc = pxs + (f & 3) * kBinW * kSub, pyc = pys + (f >> 2) * kBinH * kSub;   // this lane's pixel, coarse-relative
             bool px_valid = true;
-            if (kFish) {   // the source pixel of this lane's output pixel (lanes past the image edge read a clamped entry)
-              const int gx = min(bx * kBinW + (lane & 7), W - 1), gy = min(by * kBinH + (lane >> 3), H - 1);
-              const int sxy = __ldg(ft.src_xy + gy * W + gx);
-              const int sx = (int)(short)(sxy & 0xffff), sy = sxy >> 16;
-              px_valid = sx != -32768;
-              pxc = sx * kSub - ox; pyc = sy * kSub - oy;
+            if (kFish) {   // the source pixel of this lane's output pixel
+              const FishSrc s = fish_src(ft, bx * kBinW + (lane & 7), by * kBinH + (lane >> 3), W, H);
+              px_valid = s.valid;
+              pxc = s.x - ox; pyc = s.y - oy;
             }
             const bool live = (mine.x >> (16 + f)) & 1u;
             const unsigned live_mask = __ballot_sync(0xffffffffu, live);
@@ -1599,7 +1503,7 @@ k_raster(const DState S, const DMap* __restrict__ maps, RenderCfg rc, FrameMem f
             // two neighbours snapped their shared border differently) disjoint, so a sample belongs to the one tile that
             // covers it — no depth arithmetic; the ground lies below them and takes what is left.  A sample that turns
             // out to be covered twice sends the whole bin through the depth-tested path (exactly the spec's answer).
-            bool coplanar = DTS_COPLANAR && single && !(live_mask & ~ground_mask & ~flat_bits);
+            bool coplanar = single && !(live_mask & ~ground_mask & ~flat_bits);
             if (coplanar && !simple) DTS_COUNT(20, 1);
             if (!simple) {
               if (first) {
@@ -1820,8 +1724,8 @@ k_raster(const DState S, const DMap* __restrict__ maps, RenderCfg rc, FrameMem f
 // lean loop gets its own register allocation (the same fast path inside k_raster cost more than it saved).
 // Packed u8 HWC output with whole-word rows only (k_bin marks no bin otherwise).  Runs before k_raster.
 template <bool kFish>   // true: each lane shades the source pixel the fisheye LUT names for its output pixel
-__global__ void __launch_bounds__(256, DTS_SOLO_MIN_CTAS) k_raster_solo(const DState S, const DMap* __restrict__ maps, RenderCfg rc, FrameMem fm,
-                                                                        FishTab ft, uint8_t* __restrict__ obs, int max_prims, int max_lat) {
+__global__ void __launch_bounds__(256, kSoloMinCtas) k_raster_solo(const DState S, const DMap* __restrict__ maps, RenderCfg rc, FrameMem fm,
+                                                                   FishTab ft, uint8_t* __restrict__ obs, int max_prims, int max_lat) {
   const int W = rc.width, H = rc.height;
   const int cbins_x = (W + kCoarseW - 1) / kCoarseW;
   const int lane = threadIdx.x & 31;
@@ -1838,8 +1742,7 @@ __global__ void __launch_bounds__(256, DTS_SOLO_MIN_CTAS) k_raster_solo(const DS
     const float4* lat_tab = fm.lat + (size_t)env * max_lat * 64;
     const ShadeIn si = load_shade(fm.prims + (size_t)env * max_prims, p);
     uint8_t* out = obs + (size_t)env * frame_bytes;
-    const int nx = min(kCFX, (W - cbx * kCoarseW + kBinW - 1) / kBinW);
-    const int ny = ((cby * kCFY + 1) * kBinH < H) ? 2 : 1;
+    const int nx = fine_cols_in_image(cbx, W), ny = fine_row_mask(cby, H) == 0xffu ? 2 : 1;   // the fine bins of fine_bins_inside
 #pragma unroll 1
     for (int fy = 0; fy < ny; fy++)
 #pragma unroll 1
@@ -1847,12 +1750,10 @@ __global__ void __launch_bounds__(256, DTS_SOLO_MIN_CTAS) k_raster_solo(const DS
         const int bx = cbx * kCFX + fx, by = cby * kCFY + fy;
         int pxa = (bx * kBinW + (lane & 7)) * kSub, pya = (by * kBinH + (lane >> 3)) * kSub;
         bool px_valid = true;
-        if (kFish) {   // (lanes past the image edge read a clamped entry; their pixels are not stored)
-          const int gx = min(bx * kBinW + (lane & 7), W - 1), gy = min(by * kBinH + (lane >> 3), H - 1);
-          const int sxy = __ldg(ft.src_xy + gy * W + gx);
-          const int sx = (int)(short)(sxy & 0xffff), sy = sxy >> 16;
-          px_valid = sx != -32768;
-          pxa = sx * kSub; pya = sy * kSub;
+        if (kFish) {
+          const FishSrc s = fish_src(ft, bx * kBinW + (lane & 7), by * kBinH + (lane >> 3), W, H);
+          px_valid = s.valid;
+          pxa = s.x; pya = s.y;
         }
         float c3[3];
         shade_eval(si, tex_pool, lat_tab, pxa, pya, c3);
@@ -1870,7 +1771,13 @@ __global__ void __launch_bounds__(256, DTS_SOLO_MIN_CTAS) k_raster_solo(const DS
 // 8-bit bicubic is fixed point: per output column / row four int16 taps = cvRound(2048 * w_k(frac)), w = the a = -0.75
 // cubic kernel evaluated in float32 at frac = (d + 0.5) * scale - 0.5 - floor(.), source indices clamped to the
 // image; horizontal pass in int32, then (sum_k beta_k * row_k + 2^21) >> 22, saturated.  The tap tables are built on
-// the host (dts_set_resize).  One thread per output pixel (3 channels); reads the full-size u8 HWC render.
+// the host (dts_set_resize, cubic_axis_table), one int4 per output column / row: 4 int16 source indices, then the 4
+// int16 taps, unpacked by unpack_taps.  One thread per output pixel (3 channels); reads the full-size u8 HWC render.
+struct Taps { int i[4], w[4]; };
+__device__ __forceinline__ Taps unpack_taps(int4 t) {
+  return {{(short)(t.x & 0xffff), t.x >> 16, (short)(t.y & 0xffff), t.y >> 16},
+          {(short)(t.z & 0xffff), t.z >> 16, (short)(t.w & 0xffff), t.w >> 16}};
+}
 __global__ void __launch_bounds__(256) k_resize(const uint8_t* __restrict__ src, int W, int H, int ow, int oh, int n_envs,
                                                 const int16_t* __restrict__ xtab /*[ow][8]: 4 indices, 4 taps*/,
                                                 const int16_t* __restrict__ ytab /*[oh][8]*/, void* __restrict__ dst, int layout,
@@ -1879,23 +1786,20 @@ __global__ void __launch_bounds__(256) k_resize(const uint8_t* __restrict__ src,
   for (size_t g = blockIdx.x * (size_t)blockDim.x + threadIdx.x; g < total; g += (size_t)gridDim.x * blockDim.x) {
     const int x = (int)(g % ow), y = (int)((g / ow) % oh);
     const size_t env = g / ((size_t)ow * oh);
-    const int4 xa = __ldg(reinterpret_cast<const int4*>(xtab + 8 * x)), ya = __ldg(reinterpret_cast<const int4*>(ytab + 8 * y));
-    const int xi[4] = {(short)(xa.x & 0xffff), xa.x >> 16, (short)(xa.y & 0xffff), xa.y >> 16};
-    const int xw[4] = {(short)(xa.z & 0xffff), xa.z >> 16, (short)(xa.w & 0xffff), xa.w >> 16};
-    const int yi[4] = {(short)(ya.x & 0xffff), ya.x >> 16, (short)(ya.y & 0xffff), ya.y >> 16};
-    const int yw[4] = {(short)(ya.z & 0xffff), ya.z >> 16, (short)(ya.w & 0xffff), ya.w >> 16};
+    const Taps xt = unpack_taps(__ldg(reinterpret_cast<const int4*>(xtab + 8 * x)));
+    const Taps yt = unpack_taps(__ldg(reinterpret_cast<const int4*>(ytab + 8 * y)));
     const uint8_t* frame = src + env * (size_t)W * H * 3;
     long long acc[3] = {0, 0, 0};
 #pragma unroll
     for (int r = 0; r < 4; r++) {
-      const uint8_t* row = frame + (size_t)yi[r] * W * 3;
+      const uint8_t* row = frame + (size_t)yt.i[r] * W * 3;
       int h0 = 0, h1 = 0, h2 = 0;
 #pragma unroll
       for (int c = 0; c < 4; c++) {
-        const uint8_t* px = row + xi[c] * 3;
-        h0 += (int)px[0] * xw[c]; h1 += (int)px[1] * xw[c]; h2 += (int)px[2] * xw[c];
+        const uint8_t* px = row + xt.i[c] * 3;
+        h0 += (int)px[0] * xt.w[c]; h1 += (int)px[1] * xt.w[c]; h2 += (int)px[2] * xt.w[c];
       }
-      acc[0] += (long long)h0 * yw[r]; acc[1] += (long long)h1 * yw[r]; acc[2] += (long long)h2 * yw[r];
+      acc[0] += (long long)h0 * yt.w[r]; acc[1] += (long long)h1 * yt.w[r]; acc[2] += (long long)h2 * yt.w[r];
     }
     unsigned rgb = 0;
 #pragma unroll
@@ -1958,16 +1862,14 @@ __global__ void __launch_bounds__(256) k_resize_band(const uint8_t* __restrict__
   // horizontal pass: a warp per source row, a lane per output column (no index divisions), three channels
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
   for (int x = lane; x < ow; x += 32) {
-    const int4 xa = xt[x];
-    const int xi[4] = {(short)(xa.x & 0xffff), xa.x >> 16, (short)(xa.y & 0xffff), xa.y >> 16};
-    const int xw[4] = {(short)(xa.z & 0xffff), xa.z >> 16, (short)(xa.w & 0xffff), xa.w >> 16};
+    const Taps xa = unpack_taps(xt[x]);
     for (int row = warp; row < nrows; row += nwarps) {
       const uint8_t* rp = sb + row * rowb;
       int h0 = 0, h1 = 0, h2 = 0;
 #pragma unroll
       for (int c = 0; c < 4; c++) {
-        const uint8_t* px = rp + xi[c] * 3;
-        h0 += (int)px[0] * xw[c]; h1 += (int)px[1] * xw[c]; h2 += (int)px[2] * xw[c];
+        const uint8_t* px = rp + xa.i[c] * 3;
+        h0 += (int)px[0] * xa.w[c]; h1 += (int)px[1] * xa.w[c]; h2 += (int)px[2] * xa.w[c];
       }
       int* hp = hb + row * ow3 + x * 3;
       hp[0] = h0; hp[1] = h1; hp[2] = h2;
@@ -1981,17 +1883,15 @@ __global__ void __launch_bounds__(256) k_resize_band(const uint8_t* __restrict__
   if (words) {
     const int wpr = ow3 / 4;   // words per output row
     for (int y = r0 + warp; y < r1; y += nwarps) {   // a warp per output row, a lane per word of four bytes
-      const int4 ya = __ldg(reinterpret_cast<const int4*>(ytab) + y);
-      const int yi[4] = {(short)(ya.x & 0xffff), ya.x >> 16, (short)(ya.y & 0xffff), ya.y >> 16};
-      const int yw[4] = {(short)(ya.z & 0xffff), ya.z >> 16, (short)(ya.w & 0xffff), ya.w >> 16};
+      const Taps ya = unpack_taps(__ldg(reinterpret_cast<const int4*>(ytab) + y));
       for (int j = lane; j < wpr; j += 32) {
         const int e = 4 * j;
         // int32 like OpenCV's own vertical pass (|sum| <= 255 * sum|xw| * sum|yw| < 2^31 for cubic taps: 255 * 2621^2 = 1.75e9)
         int acc[4] = {0, 0, 0, 0};
 #pragma unroll
         for (int r = 0; r < 4; r++) {
-          const int4 hv = *reinterpret_cast<const int4*>(hb + (yi[r] - s_lo) * ow3 + e);
-          acc[0] += hv.x * yw[r]; acc[1] += hv.y * yw[r]; acc[2] += hv.z * yw[r]; acc[3] += hv.w * yw[r];
+          const int4 hv = *reinterpret_cast<const int4*>(hb + (ya.i[r] - s_lo) * ow3 + e);
+          acc[0] += hv.x * ya.w[r]; acc[1] += hv.y * ya.w[r]; acc[2] += hv.z * ya.w[r]; acc[3] += hv.w * ya.w[r];
         }
         unsigned word = 0;
 #pragma unroll
@@ -2005,12 +1905,10 @@ __global__ void __launch_bounds__(256) k_resize_band(const uint8_t* __restrict__
   } else {
     for (int i = threadIdx.x; i < (r1 - r0) * ow3; i += blockDim.x) {
       const int yy = i / ow3, e = i - yy * ow3, y = r0 + yy, x = e / 3, ch = e - 3 * x;
-      const int4 ya = __ldg(reinterpret_cast<const int4*>(ytab) + y);
-      const int yi[4] = {(short)(ya.x & 0xffff), ya.x >> 16, (short)(ya.y & 0xffff), ya.y >> 16};
-      const int yw[4] = {(short)(ya.z & 0xffff), ya.z >> 16, (short)(ya.w & 0xffff), ya.w >> 16};
+      const Taps ya = unpack_taps(__ldg(reinterpret_cast<const int4*>(ytab) + y));
       long long acc = 0;
 #pragma unroll
-      for (int r = 0; r < 4; r++) acc += (long long)hb[(yi[r] - s_lo) * ow3 + e] * yw[r];
+      for (int r = 0; r < 4; r++) acc += (long long)hb[(ya.i[r] - s_lo) * ow3 + e] * ya.w[r];
       long long v = (acc + (1LL << 21)) >> 22;
       v = v < 0 ? 0 : (v > 255 ? 255 : v);
       const size_t oi = fmt_index(layout, x, y, ch, ow, oh);
@@ -2093,15 +1991,14 @@ int launch_render(const DState& S, const DMap* maps, const RenderCfg& rc, void* 
   mark();
   const size_t pairs_total = (size_t)rc.n_envs * items_max;
   k_cull<<<(unsigned)((pairs_total + 255) / 256), 256, 0, st>>>(S, maps, rc, fm, items_max);
-  const int geo_ctas = (n_ctas / DTS_RENDER_MIN_CTAS) * DTS_GEO_MIN_CTAS / kGeoWarps;   // SMs x resident geometry CTAs
+  const int geo_ctas = (n_ctas / kRenderMinCtas) * kGeoMinCtas / kGeoWarps;   // SMs x resident geometry CTAs
   if (rc.tessellate) k_geometry<true><<<geo_ctas, kGeoWarps * 32, 0, st>>>(S, maps, rc, fm, max_prims, max_lat, err_flag);
   else k_geometry<false><<<geo_ctas, kGeoWarps * 32, 0, st>>>(S, maps, rc, fm, max_prims, max_lat, err_flag);
   mark();
   const size_t bin_smem_bytes = (size_t)2 * cbins * sizeof(int);
   const int bin_grid = rc.n_envs;   // CTA per env: one warp where a frame has few bins and prims (160x120: 75 bins — more warps
   // only add barriers and CTA launches, measured 58 -> 88 us), four for large cameras (640x480: 9.0 -> 3.3 ms)
-  static const int bin_warps_env = getenv("DTS_BIN_WARPS") ? atoi(getenv("DTS_BIN_WARPS")) : 0;   // A/B override: 1..4
-  const int bin_threads = bin_warps_env >= 1 && bin_warps_env <= kBinWarps ? bin_warps_env * 32 : (cbins > 128 ? kBinWarps * 32 : 32);
+  const int bin_threads = cbins > 128 ? kBinWarps * 32 : 32;
   if (fisheye) {
     if (bin_smem_bytes > 48 * 1024) cudaFuncSetAttribute(k_bin<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bin_smem_bytes);
     k_bin<true><<<bin_grid, bin_threads, bin_smem_bytes, st>>>(rc, fm, fish, max_prims, max_pairs, err_flag);
@@ -2113,8 +2010,8 @@ int launch_render(const DState& S, const DMap* maps, const RenderCfg& rc, void* 
   mark();
   const bool wrap = (rc.obs_layout | rc.obs_dtype) != 0;
   int launches = 5;
-  if (DTS_SOLO && !wrap && (W & 3) == 0) {   // (inside the k_raster event bracket: it is rasterisation time)
-    const int solo_ctas = max(1, n_ctas * DTS_SOLO_MIN_CTAS / DTS_RENDER_MIN_CTAS);   // (n_ctas can be 1 for a handful of envs)
+  if (!wrap && (W & 3) == 0) {   // (inside the k_raster event bracket: it is rasterisation time)
+    const int solo_ctas = max(1, n_ctas * kSoloMinCtas / kRenderMinCtas);   // (n_ctas can be 1 for a handful of envs)
     if (fisheye) k_raster_solo<true><<<solo_ctas, 256, 0, st>>>(S, maps, rc, fm, fish, obs, max_prims, max_lat);
     else k_raster_solo<false><<<solo_ctas, 256, 0, st>>>(S, maps, rc, fm, fish, obs, max_prims, max_lat);
     launches++;

@@ -147,7 +147,7 @@ def load() -> C.CDLL:
         return _lib
     import shutil
     from . import build as _b
-    if os.environ.get("DTS_NO_REBUILD"):     # A/B runs of pre-built variants (tools/ab_all.sh): load what is there
+    if os.environ.get("DTS_NO_REBUILD"):     # load the library as built (e.g. a -DDTS_STATS build), never rebuild it
         pass
     elif shutil.which("nvcc"):
         _b.build(force=False)

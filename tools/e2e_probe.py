@@ -1,6 +1,6 @@
 """Where does the end-to-end time go?  Device-only stepping vs HostPipeline at several depths, full size and 84x84."""
-import sys, time, torch
-sys.path.insert(0, "/root/repo")
+import os, sys, time, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from collections import deque
 from gym_duckietown_b200.batched_env import BatchedDuckietownEnv, HostPipeline
 N, K = 4096, 60

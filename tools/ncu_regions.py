@@ -1,6 +1,6 @@
 """Instruction / sample shares of k_raster by source region (line ranges found by marker comments in dts_render.cu)."""
-import csv, sys, re
-src = open('/root/repo/gym-duckietown_b200/csrc/dts_render.cu').read().splitlines()
+import csv, os, sys, re
+src = open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'gym-duckietown_b200', 'csrc', 'dts_render.cu')).read().splitlines()
 def find(pat, start=0):
     for i in range(start, len(src)):
         if pat in src[i]: return i + 1

@@ -1,6 +1,11 @@
-"""Print DTS_STATS counters of the raster kernel for the bench workload (needs a -DDTS_STATS build)."""
-import sys, torch, numpy as np
-sys.path.insert(0, "/root/repo")
+"""Print DTS_STATS counters of the raster kernel for the bench workload (needs a -DDTS_STATS build):
+
+    DTS_NVCC_EXTRA=-DDTS_STATS=1 python gym-duckietown_b200/build.py --force
+    python tools/raster_stats.py [map]
+    python gym-duckietown_b200/build.py --force    # back to the product build
+"""
+import os, sys, torch, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from gym_duckietown_b200.batched_env import BatchedDuckietownEnv
 m = sys.argv[1] if len(sys.argv) > 1 else "small_loop"
 env = BatchedDuckietownEnv(4096, m, camera_width=160, camera_height=120, domain_rand=False, seed=1000, auto_reset=True, device_reset=True)

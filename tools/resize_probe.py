@@ -1,6 +1,6 @@
-"""Device-only step time with the device ResizeWrapper under the current DTS_RESIZE_* switches (A/B of k_resize_band)."""
-import sys, time, torch
-sys.path.insert(0, "/root/repo")
+"""Device-only step time at full size and with the device ResizeWrapper to 84x84: what the resize costs per step."""
+import os, sys, time, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from gym_duckietown_b200.batched_env import BatchedDuckietownEnv
 N, K = 4096, 60
 env = BatchedDuckietownEnv(N, "small_loop", camera_width=160, camera_height=120, seed=1000, auto_reset=True, device_reset=True)

@@ -1,7 +1,7 @@
 """A small tour of every kernel for compute-sanitizer (memcheck / racecheck / initcheck): meshes, fisheye at 640x480,
 wrapper layouts, the device resize, device resets, the literal tile mode."""
-import sys, torch
-sys.path.insert(0, "/root/repo")
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from gym_duckietown_b200.batched_env import BatchedDuckietownEnv
 def run(n, m, w, h, steps=3, fmt=None, resize=None, **kw):
     env = BatchedDuckietownEnv(n, m, camera_width=w, camera_height=h, seed=3, auto_reset=True, device_reset=True, **kw)

@@ -1,6 +1,7 @@
 """Triangle statistics of the raster oracle (orr_stats_read) for a few maps: how many set-up triangles reach no sample."""
-import sys, numpy as np, ctypes as C
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/oracle')
+import os, sys, numpy as np, ctypes as C
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'oracle'))
 import oracle as orc
 from gym_duckietown_b200 import maps
 orc.build(force=True)
